@@ -3,6 +3,12 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR
+
+--dump-outputs DIR writes what the last timed step computed, as a caller of tsb_energy_grad receives it:
+DIR/energy.npy (float32 [3]: total, smoothness, barrier) and DIR/grad.npy (float32 [n,3]); under torchrun
+every rank writes its own, suffixed _rank<r>.  The inputs depend on the arguments only, so two builds run
+with the same arguments can be compared file by file.
 
 A *step* is ONE launch of the fused energy+gradient kernel (tsb_energy_grad) over one synthetic pack
 of 64 tet-spheres x 4096 tets (BASELINE.json metric; the kernel-only form of configs[2], whose
@@ -52,6 +58,7 @@ METRIC = "geometry_energy_grad_iters_per_sec_64x4k"
 UNIT = "iters/s"
 N_ROTATE = 8           # distinct packs per rank; 8 x ~23 MB of plan data > 126 MB L2
 ORDER = 2
+DUMP_BYTES = 64 << 20  # --dump-outputs budget over all ranks; a larger gradient is written as a seeded row sample
 KERNEL_SOURCES = ("tssplat_b200/csrc/tsb_kernels.cu", "tssplat_b200/csrc/tsb_plan.cpp", "tssplat_b200/csrc/tsb_plan.h")
 
 
@@ -220,6 +227,17 @@ def run_reference(args):
 
 
 # ---- GPU arm ---------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, energy, grad, suffix="", budget=DUMP_BYTES):
+    """energy[3] and grad[n,3] (host float32) as out_dir/energy<suffix>.npy and grad<suffix>.npy.  A gradient larger
+    than the budget keeps a fixed, seeded, sorted sample of its rows, the same one for every build."""
+    os.makedirs(out_dir, exist_ok=True)
+    if grad.nbytes + energy.nbytes > budget:
+        keep = (budget - energy.nbytes) // grad[0].nbytes
+        grad = grad[np.sort(np.random.default_rng(0).choice(len(grad), keep, replace=False))]
+    np.save(os.path.join(out_dir, f"energy{suffix}.npy"), energy)
+    np.save(os.path.join(out_dir, f"grad{suffix}.npy"), grad)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -233,7 +251,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--min-seconds", type=float, default=2.0, help="CPU arm: minimum timed duration")
     ap.add_argument("--no-extras", action="store_true", help="skip the size sweep / trainer-loop / strong-scaling extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the energy and gradient of the last timed step to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)
@@ -372,6 +393,11 @@ def main():
     sampler.start()
     t_local = timed_region(args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs:       # before anything else launches on these buffers
+        rem = args.steps % graph_len
+        last = (rem - 1 if rem else graph_len - 1) % n_rotate          # pack of the last timed step
+        dump_outputs(args.dump_outputs, energies[last].cpu().numpy(), grads[last].cpu().numpy(),
+                     f"_rank{rank}" if world > 1 else "", DUMP_BYTES // world)
     t_all = torch.tensor([t_local], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t_all, op=dist.ReduceOp.MAX)

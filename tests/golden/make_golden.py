@@ -1,9 +1,11 @@
-"""Generates the committed golden fixtures.  Run HERE (needs /root/reference for a.veg):
+"""Generates the committed golden fixtures from the original project's ``tssplat_ext/a.veg``:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <original project>/tssplat_ext/a.veg
 
 * ``a_veg_mesh.npz``  -- the reference's only in-tree tet mesh (``tssplat_ext/a.veg``: 4500 verts,
-  22120 tets) converted to arrays, so GPU-box tests can use it (``/root/reference`` is absent there).
+  22120 tets) converted to arrays, so the tests can use it without the original project.
+* ``a_veg_excerpt.veg`` -- the first 1000 vertex lines of ``a.veg`` and the element lines among them, verbatim,
+  with the header counts adjusted: a small sample of the reference's own file for the ``.veg`` reader.
 * ``golden_energy.npz`` -- energies and gradient checksums produced by the fp64 sparse-operator
   oracle (``oracle/tet_energy_oracle.py``, restating ``tet_spheres_cuda.cu:118-263``) on seeded
   inputs.  The reference ships NO golden vectors for this path and cannot be built here (libpgo),
@@ -45,8 +47,22 @@ def run(mesh_name, verts, tets, out):
         print(key, float(out[key + "/energy"]), float(out[key + "/inverted_fraction"]))
 
 
+def write_veg_excerpt(src, dst, n_verts=1000):
+    """Vertex lines 1..n_verts of ``src`` and the element lines whose four vertices are among them, verbatim."""
+    lines = open(src).read().splitlines()
+    iv, ie = lines.index("*VERTICES"), lines.index("*ELEMENTS")
+    assert lines[ie + 1] == "TET" and int(lines[iv + 1].split()[0]) >= n_verts
+    ne = int(lines[ie + 2].split()[0])
+    elems = [ln for ln in lines[ie + 3:ie + 3 + ne] if max(int(s) for s in ln.split()[1:5]) <= n_verts]
+    with open(dst, "w") as f:
+        f.write("\n".join([lines[0], f"# {n_verts} vertices, {len(elems)} elements", "", "*VERTICES", f"{n_verts} 3 0 0",
+                           *lines[iv + 2:iv + 2 + n_verts], "", "*ELEMENTS", "TET", f"{len(elems)} 4 0", *elems,
+                           *lines[ie + 3 + ne:]]) + "\n")
+
+
 if __name__ == "__main__":
-    v, t = load_veg("/root/reference/tssplat_ext/a.veg")
+    write_veg_excerpt(sys.argv[1], os.path.join(HERE, "a_veg_excerpt.veg"))
+    v, t = load_veg(sys.argv[1])
     np.savez_compressed(os.path.join(HERE, "a_veg_mesh.npz"), verts=v.astype(np.float64), tets=t.astype(np.int32))
     out = {}
     run("a_veg", v, t, out)

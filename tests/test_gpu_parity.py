@@ -378,6 +378,32 @@ def test_bench_input_and_config4_parity(ext):
     assert sp.info["n_components"] == 1024
 
 
+def test_bench_dump_outputs(ext, tmp_path):
+    """bench.py --dump-outputs: the energy and gradient of the last timed step (one step: the first pack), equal to the
+    fp64 C oracle on that pack's input, bitwise the same in a second run, and exactly --steps timed launches."""
+    import json
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    S = 64                                                             # bench.py's default pack
+    for run in ("a", "b"):
+        cmd = [sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "1", "--warmup", "3",
+               "--no-extras", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / run)]
+        r = subprocess.run(cmd, capture_output=True, text=True, timeout=900)
+        assert r.returncode == 0, r.stderr[-2000:]
+        d = json.loads(r.stdout.strip().splitlines()[-1])
+        assert d["steps"] == 1 and d["gpu_launches"] == 1
+    e, g = np.load(tmp_path / "a" / "energy.npy"), np.load(tmp_path / "a" / "grad.npy")
+    assert e.dtype == np.float32 and e.shape == (3,) and g.dtype == np.float32
+    assert np.array_equal(e, np.load(tmp_path / "b" / "energy.npy")) and np.array_equal(g, np.load(tmp_path / "b" / "grad.npy"))
+    pack = make_pack(S, 4096, seed=0, unique=8)                       # bench.py: rank 0, pack 0
+    x_np = perturb(pack, sigma_rel=0.02, seed=0)
+    eo, terms, go = COracle(pack.verts, pack.tets).energy_grad(x_np, 2e-4 / S, 2e-4, 2)
+    assert g.shape == (pack.n, 3)
+    assert abs(float(e[0]) - eo) <= REL * abs(eo) and abs(float(e[1]) - terms[0]) <= REL * abs(terms[0])
+    assert np.linalg.norm(g.astype(np.float64) - go) <= REL * np.linalg.norm(go)
+
+
 def test_reference_pinned_barrier_and_F(ext):
     """Fixtures computed by the reference's own compute_G_matrix (geometry/mesh_utils.py:38-69, imported by
     tests/golden/make_ref_fixtures.py): the kernel's barrier sum equals sum max(-det F_ref, 0)^p."""
