@@ -153,6 +153,41 @@ int tsb_adam_uniform_step(float *p_dev, const float *grad_dev, float *g1_dev, fl
                           int64_t count, double lr, double beta1, double beta2, int32_t step,
                           double grad_limit, float *work_dev, void *stream);
 
+/* State of tsb_train_step.  All buffers are caller-owned device memory on the handle's device.  The schedule row of
+ * step k (0-based, k = *step) holds what the reference's loop changes on every step (trainer.py:71-132,
+ * energies/smooth_barrier.py:47-63, utils/optimizer.py:37-89), each computed in double on the host and rounded to
+ * float: the coefficient multiplier m of coeff_scheduler, the learning rate, the two bias corrections
+ * 1/(1-beta^(k+1)) and the grad_limit value (<= 0: no clamp). */
+typedef struct {
+  float *g1, *g2;            /* [3n] Adam moments (zero-initialised by the caller), as AdamUniform's state g1, g2      */
+  float *grad;               /* [3n] scratch: the energy gradient of the fused launch                              */
+  float *energy;             /* [4]  scratch: energy_out of the fused launch                                       */
+  const float *schedule;     /* [n_steps][5]: m, lr, 1/(1-b1^t), 1/(1-b2^t), grad_limit                            */
+  float *history;            /* [n_steps][4]: loss = m * energy[0], smoothness, barrier, m; row k written by step k */
+  int32_t *step;             /* device counter: steps taken = schedule row of the next step (zero it to start)     */
+  float *work;               /* [8] scratch, zero-initialised once.  [0..2] are left zeroed by every step; [3] != 0
+                                records that a step ran with *step >= n_steps (it then left everything untouched)   */
+  int32_t n_steps;
+  double beta1, beta2;       /* Adam betas (1 - beta is formed in double, like the reference's Python)             */
+} tsb_train_state_t;
+
+/* One step of the reference's geometry loop: the fused energy + gradient launch with the base coefficients c1, c2
+ * (gradH = 1) into st->grad / st->energy, then g = m * grad (+ grad_ext_dev, e.g. the image loss's gradient of the
+ * vertex positions; may be NULL) and AdamUniform with the schedule row *step, which updates x_dev, g1, g2 in place,
+ * writes history[*step] and increments *step -- three launches (four in global-gather mode), no host sync, no
+ * host-side state that changes between calls.  coeff_scheduler scales c1 and c2 by the same m, so m multiplies the
+ * gradient (and the energy in the history) instead of the coefficients.  The barrier order is an argument: it
+ * changes once (smooth_barrier.py:61-63), so a caller records one sequence per order.
+ * Replaces, per step: SmoothnessBarrierFunc forward + backward (energies/smooth_barrier.py:9-31,60-67),
+ * coeff_scheduler (:47-58), AdamUniform.step (utils/optimizer.py:37-89) and the LR scheduler step
+ * (trainer.py:57-58,128-133).
+ * Safe to capture in a CUDA graph: every per-step value is read on the device.  Inside a graph x_dev, grad_ext_dev
+ * and the state's pointers are the ones given at capture time (rewrite the buffers' contents, not the pointers).
+ * One launch may be in flight per handle, as for tsb_energy_grad.  work holds a ticket: one state per concurrently
+ * used stream. */
+int tsb_train_step(tsb_handle_t h, float *x_dev, const float *grad_ext_dev, float c1, float c2, int32_t order,
+                   const tsb_train_state_t *st, void *stream);
+
 /* ---- "Next" row (f)2: surface gather + vertex-normal splat ------------------------------------------------
  * Replaces `tet_v[surface_vid]` (geometry/tetmesh_geometry.py:33) and `_compute_vertex_normal`
  * (geometry/tetmesh_geometry.py:39-66) and their autograd backward.  surface_vid: host int32 [nsv] tet-mesh

@@ -18,7 +18,7 @@ TSB_OK, TSB_E_INVALID, TSB_E_MESH, TSB_E_CUDA, TSB_E_NOMEM = 0, -1, -2, -3, -4
 # every symbol include/tssplat_b200.h declares (tests check the library exports each one)
 EXPORTED_SYMBOLS = (
     "tsb_create", "tsb_destroy", "tsb_last_error", "tsb_get_info", "tsb_energy_grad", "tsb_energy_grad_ex", "tsb_energy_grad_host", "tsb_scale",
-    "tsb_grad_limit", "tsb_adam_uniform_step",
+    "tsb_grad_limit", "tsb_adam_uniform_step", "tsb_train_step",
     "tsb_surface_create", "tsb_surface_destroy", "tsb_surface_last_error", "tsb_surface_forward", "tsb_surface_backward",
     "tsb_surface_extract", "tsb_free_host", "tsb_setup_last_error",
 )
@@ -41,6 +41,12 @@ class tsb_info_t(C.Structure):
         ("n_boundary_faces", C.c_int32), ("max_component_vertices", C.c_int32),
         ("nnz", C.c_int64), ("nnz_padded", C.c_int64), ("device_bytes", C.c_int64), ("stream_bytes", C.c_int64),
     ]
+
+
+class tsb_train_state_t(C.Structure):
+    _fields_ = [("g1", C.c_void_p), ("g2", C.c_void_p), ("grad", C.c_void_p), ("energy", C.c_void_p),
+                ("schedule", C.c_void_p), ("history", C.c_void_p), ("step", C.c_void_p), ("work", C.c_void_p),
+                ("n_steps", C.c_int32), ("beta1", C.c_double), ("beta2", C.c_double)]
 
 
 def _load() -> C.CDLL:
@@ -73,6 +79,8 @@ def _load() -> C.CDLL:
     lib.tsb_grad_limit.argtypes = [vp, i64, f32, f32, vp, vp]
     lib.tsb_adam_uniform_step.restype = C.c_int
     lib.tsb_adam_uniform_step.argtypes = [vp, vp, vp, vp, i64, C.c_double, C.c_double, C.c_double, i32, C.c_double, vp, vp]
+    lib.tsb_train_step.restype = C.c_int
+    lib.tsb_train_step.argtypes = [vp, vp, vp, f32, f32, i32, C.POINTER(tsb_train_state_t), vp]
     lib.tsb_surface_create.restype = C.c_int
     lib.tsb_surface_create.argtypes = [vp, i32, vp, i32, i32, C.c_int, C.POINTER(vp)]
     lib.tsb_surface_destroy.restype = None

@@ -13,7 +13,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.path.join(HERE, "libtssplat_b200.so")
-SOURCES = ["tsb_plan.cpp", "tsb_kernels.cu", "tsb_capi.cu", "tsb_surface.cu", "tsb_setup.cu"]
+SOURCES = ["tsb_plan.cpp", "tsb_kernels.cu", "tsb_capi.cu", "tsb_surface.cu", "tsb_setup.cu", "tsb_train.cu"]
 HEADERS = ["tsb_plan.h", "tsb_kernels.cuh", os.path.join("..", "..", "include", "tssplat_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

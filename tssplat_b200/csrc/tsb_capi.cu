@@ -396,6 +396,26 @@ int tsb_adam_uniform_step(float *p_dev, const float *grad_dev, float *g1_dev, fl
   return TSB_OK;
 }
 
+int tsb_train_step(tsb_handle_t h, float *x_dev, const float *grad_ext_dev, float c1, float c2, int32_t order,
+                   const tsb_train_state_t *st, void *stream) {
+  if (!h) return TSB_E_INVALID;
+  if (!x_dev || !st) return fail(h, TSB_E_INVALID, "tsb_train_step: x_dev and st must be non-null");
+  if (!st->g1 || !st->g2 || !st->grad || !st->energy || !st->schedule || !st->history || !st->step || !st->work)
+    return fail(h, TSB_E_INVALID, "tsb_train_step: a state buffer is null");
+  if (st->n_steps < 1) return fail(h, TSB_E_INVALID, "tsb_train_step: n_steps must be >= 1");
+  if (!(st->beta1 >= 0.0 && st->beta1 < 1.0 && st->beta2 >= 0.0 && st->beta2 < 1.0))
+    return fail(h, TSB_E_INVALID, "tsb_train_step: betas must be in [0, 1)");
+  // validates order, selects the device and runs the very launch tsb_energy_grad runs with gradH = 1
+  int rc = energy_grad_impl(h, x_dev, c1, c2, 0.f, order, 1.f, nullptr, st->energy, 0, st->grad, stream);
+  if (rc != TSB_OK) return rc;
+  DeviceGuard guard(h->device);
+  cudaError_t e = tsb::launch_train_adam(x_dev, st->grad, grad_ext_dev, st->g1, st->g2, int64_t(h->info.n) * 3, st->beta1,
+                                         st->beta2, st->schedule, st->energy, st->history, st->step, st->n_steps, st->work,
+                                         static_cast<cudaStream_t>(stream));
+  if (e != cudaSuccess) return fail(h, TSB_E_CUDA, std::string("train_step launch: ") + cudaGetErrorString(e));
+  return TSB_OK;
+}
+
 #ifdef TSB_TRACE
 /* profiling build only: copy the [grid][16] phase stamps of the last launch to the host */
 int tsb_trace_read(tsb_handle_t h, unsigned long long *out, int64_t count) {

@@ -68,4 +68,11 @@ cudaError_t launch_grad_limit(float *g, int64_t count, float thr, float s, float
 cudaError_t launch_adam_uniform(float *p, const float *grad, float *g1, float *g2, int64_t count, double lr,
                                 double b1, double b2, int step, double grad_limit, float *work4, cudaStream_t st);
 
+// tsb_train.cu: the AdamUniform half of tsb_train_step (schedule row (m, lr, 1/(1-b1^t), 1/(1-b2^t), grad_limit)
+// selected by *step).  work: [0..1] the two maxima, [2] the ticket, [kTrainWorkFlag] set when *step >= n_steps.
+constexpr int kTrainWorkFlag = 3;
+cudaError_t launch_train_adam(float *p, const float *grad_e, const float *grad_ext, float *g1, float *g2, int64_t count,
+                              double b1, double b2, const float *schedule, const float *energy, float *history,
+                              int32_t *step, int32_t n_steps, float *work, cudaStream_t st);
+
 }  // namespace tsb
